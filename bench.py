@@ -7,6 +7,7 @@ Default workload = BASELINE.json configs[1]: Mistral-7B full (32 layers, GQA 32/
     python bench.py --gpus N --steps K --warmup W              # this repo's CUDA path
     python bench.py --impl reference --gpus N ...               # the reference's algorithm on the host CPUs (full depth)
     python bench.py --model mistral-nemo-12b --batch 32 --prefill 1024    # BASELINE configs[2] (informational lines)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR      # + the last timed step's outputs as DIR/*.npy
     torchrun ... bench.py --gpus N --parallel expert --model mixtral-8x7b --batch 8 --prefill 2048   # configs[3]/[4]: expert-sharded
 
 Under torchrun (N > 1) the dense 7B model is "replicas only" (it fits one GPU; DESIGN.md section (e)): every rank runs the same
@@ -145,6 +146,29 @@ def whole_job_tokens_per_s(replicas: int, batch: int, steps: int, elapsed_ms: fl
     return replicas * batch * steps * 1000.0 / elapsed_ms
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: writes each tensor as out_dir/<name>.npy, floating point as float32 and token ids as float64 (exact), so
+    that two builds run with the same arguments can be compared output for output.  A tensor larger than its share of
+    DUMP_LIMIT_BYTES is replaced by a fixed seeded sample of its elements (flattened), written with their indices as
+    <name>_index.npy."""
+    import numpy as np
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    for name, t in arrays.items():
+        x = t.detach().cpu()
+        x = (x.double() if not x.is_floating_point() else x.float()).numpy()
+        if x.nbytes > share:  # a sampled element costs its own bytes + 8 for its index
+            idx = np.sort(np.random.default_rng(0).choice(x.size, share // (x.itemsize + 8), replace=False))
+            np.save(out / f"{name}_index.npy", idx.astype(np.float64))
+            x = x.reshape(-1)[idx]
+        np.save(out / f"{name}.npy", x)
+
+
 # ------------------------------------------------------------------------------------------------ our arm
 def build_gpu_model(p: dict, max_batch: int, seed: int = 0, expert_parallel=None):
     import mistral_inference_b200 as mi
@@ -174,14 +198,16 @@ def moe_stats(model, batch: int):
 
 def timed_decode(model, cache, tok, steps: int, warmup: int, world: int, dev_index: int, sample_clocks: bool = True):
     """W warm-up + K timed decode steps with the token fed back on the device.  Returns (ms total max over ranks, us per launch
-    of the hot-path launch (CUDA events on the launch stream, this rank), clocks summary, last token)."""
+    of the hot-path launch (CUDA events on the launch stream, this rank), clocks summary, last token, fp32 logits [B, V] of the
+    last step (the step's static buffer: valid until the next decode step))."""
     kern_ev = []
+    last = {}
 
     def step(t, timed=False):
         if timed:
             a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a0.record()
-            model.decode_static(t, cache)
+            last["logits"] = model.decode_static(t, cache)
             a1.record()
             kern_ev.append((a0, a1))
         else:
@@ -204,7 +230,7 @@ def timed_decode(model, cache, tok, steps: int, warmup: int, world: int, dev_ind
         torch.cuda.synchronize()
     ms = max_over_ranks(e0.elapsed_time(e1), world, torch.device("cuda", dev_index))
     kern_us = 1000.0 * sum(x.elapsed_time(y) for x, y in kern_ev) / len(kern_ev)
-    return ms, kern_us, clocks.summary() if sample_clocks else None, tok
+    return ms, kern_us, clocks.summary() if sample_clocks else None, tok, last["logits"]
 
 
 def parity_check(model, p, prompt, seqlens, steps: int):
@@ -284,6 +310,7 @@ def run_ours(a, rank: int, world: int):
     times = []
     tok = None
     cache = None
+    prefill_last = None
     for rep in range(4):
         del cache
         cache = fresh_cache()
@@ -300,6 +327,8 @@ def run_ours(a, rank: int, world: int):
         if rep:
             times.append(e0.elapsed_time(e1))
         tok = last.argmax(-1)
+        if a.dump_outputs and rep == 3:
+            prefill_last = last.float().cpu()  # after the timed region: the copy is not timed
         del last
     prefill_ms = max_over_ranks(sorted(times)[1], world, model.device)
     pf = prefill_flops(p, a.prefill) * a.batch  # the lm head runs on every row in both variants (forward_logprobs: block by block)
@@ -344,8 +373,11 @@ def run_ours(a, rank: int, world: int):
     # ---- decode: device-resident loop (value).  Runs after the end-to-end loop: the first decode steps right after the prefills of a
     # fresh process were measured up to 5 % slower than steady state on some boxes; W warm-up steps still precede the K timed ones ----
     st0 = moe_stats(model, a.batch)
-    dec_ms, kern_us, clocks, tok = timed_decode(model, cache, tok, a.steps, a.warmup, world, dev_index)
+    dec_ms, kern_us, clocks, tok, dec_logits = timed_decode(model, cache, tok, a.steps, a.warmup, world, dev_index)
     st1 = moe_stats(model, a.batch)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"decode_logits": dec_logits, "decode_next_token": tok, "prefill_last_logits": prefill_last})
+    del dec_logits
     touched = (st1[0] - st0[0]) / (st1[1] - st0[1]) if st1[1] > st0[1] else None  # measured distinct experts per MoE layer call
     ms_per_step = dec_ms / a.steps
     value = whole_job_tokens_per_s(replicas, a.batch, a.steps, dec_ms)
@@ -451,7 +483,7 @@ def run_sharded(a, rank: int, world: int, dev_index: int):
     prefill_ms = max_over_ranks(e0.elapsed_time(e1), world, model.device)
     tok = last.argmax(-1)
     st0 = moe_stats(model, B)
-    ms, kern_us, _, _ = timed_decode(model, cache, tok, K, Wm, world, dev_index, sample_clocks=False)
+    ms, kern_us, _, _, _ = timed_decode(model, cache, tok, K, Wm, world, dev_index, sample_clocks=False)
     st1 = moe_stats(model, B)
     touched = (st1[0] - st0[0]) / (st1[1] - st0[1]) if st1[1] > st0[1] else None
     peaks = measured_peaks()
@@ -588,7 +620,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed decode step returned (fp32 "
+                    "logits, greedy next token) and the last timed prefill's last-token logits as DIR/<name>.npy (at most 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))

@@ -1,8 +1,9 @@
 """Generate tests/golden/*.safetensors from the UNMODIFIED reference modules
 (TEST INFRASTRUCTURE -- see oracle/__init__.py).
 
-Run in the build container (where /root/reference exists):   python -m oracle.make_golden
-The reference cannot travel to the GPU box, so its outputs on small seeded cases are committed as
+Run where a checkout of the reference is installed (MISTRAL_REFERENCE_SRC = its src/ directory):
+    python -m oracle.make_golden [--config1 | --modules | --all]
+The tests must not need the reference, so its outputs on small seeded cases are committed as
 fixtures.  Each fixture holds the outputs of the reference's own `Transformer.forward` /
 `generate` (mistral_inference/transformer.py:221-242, generate.py:43-148) imported behind
 oracle/ref_shims.py, on weights from synth (bit-reproducible anywhere).
@@ -143,6 +144,84 @@ def run_config1(max_seeds: int = 6):
     return best[1], best[0], best[2]
 
 
+# ---- tests/test_oracle_vs_reference.py: what the reference's modules return on the inputs of each of its tests, so the restatement
+# is pinned against the reference anywhere, not only where the reference tree is installed.  The rope table (1000 x 64 complex) is
+# stored as the SHA-256 of its bytes plus a sample of rows; everything else is stored whole (about 100 KB in all).
+MODULES_FILE = GOLDEN_DIR / "reference_modules" / "outputs.safetensors"
+MODULES_GENERATE_CASES = [("tiny", {}), ("tiny", {"sliding_window": 5}), ("tiny", {"sliding_window": [4, None]}),
+                          ("tiny-moe", {}), ("tiny-moe", {"sliding_window": 3})]
+MODULES_DTYPES = [torch.bfloat16, torch.float32]
+ROPE_SAMPLE_ROWS = sorted(set(range(0, 1000, 25)) | {1, 2, 500, 501, 998, 999})
+
+
+def modules_generate_key(shape: str, over: dict, dtype: torch.dtype) -> str:
+    return f"generate/{shape}/{json.dumps(over, sort_keys=True)}/{str(dtype).removeprefix('torch.')}"
+
+
+def elementwise_inputs():
+    """The inputs of the element-wise comparison (seeded torch CPU generator; stored with the outputs)."""
+    torch.manual_seed(0)
+    x = torch.randn(7, 256).to(torch.bfloat16)
+    w = (1 + 0.1 * torch.randn(256)).to(torch.bfloat16)
+    q = torch.randn(7, 4, 128).to(torch.bfloat16)
+    k = torch.randn(7, 2, 128).to(torch.bfloat16)
+    return {"x": x, "w": w, "q": q, "k": k, "positions": torch.tensor([0, 1, 2, 500, 501, 998, 999])}
+
+
+def tensor_sha256(t: torch.Tensor) -> str:
+    import hashlib
+
+    return hashlib.sha256(t.contiguous().view(torch.uint8).numpy().tobytes()).hexdigest()
+
+
+def _ref_model(ref, p: dict, max_batch: int, dtype: torch.dtype, seed: int = 3):
+    args = ref.args.TransformerArgs.from_dict(dict(p))
+    args.max_batch_size = max_batch
+    with torch.device("meta"):
+        m = ref.transformer.Transformer(args)
+    m.load_state_dict(synth.synth_state_dict(p, seed, dtype), assign=True, strict=True)
+    return m.eval()
+
+
+def run_modules():
+    ref = ref_shims.import_reference()
+    import mistral_inference.rope as r_rope  # type: ignore
+    import mistral_inference.transformer_layers as r_layers  # type: ignore
+
+    out: Dict[str, torch.Tensor] = {}
+    for shape, over in MODULES_GENERATE_CASES:
+        for dtype in MODULES_DTYPES:
+            p = synth.shape(shape, **over)
+            rm = _ref_model(ref, p, 3, dtype)
+            prompts = [synth.synth_prompt(n, p["vocab_size"], 40 + i) for i, n in enumerate([11, 9, 10])]
+            toks, logprobs = ref.generate.generate(prompts, rm, max_tokens=9, temperature=0.0, chunk_size=4)
+            key = modules_generate_key(shape, over, dtype)
+            out[key + "/tokens"] = torch.tensor(toks, dtype=torch.int64)
+            out[key + "/logprobs"] = torch.tensor(sum(logprobs, []), dtype=torch.float64)  # python floats of fp32 values: exact
+            out[key + "/logprob_counts"] = torch.tensor([len(x) for x in logprobs], dtype=torch.int64)
+    for dtype in MODULES_DTYPES:
+        p = synth.shape("tiny")
+        rm = _ref_model(ref, p, 2, dtype)
+        toks = torch.tensor(synth.synth_prompt(13, p["vocab_size"], 5))
+        with torch.inference_mode():
+            out[f"forward_no_cache/{str(dtype).removeprefix('torch.')}"] = rm.forward(toks, seqlens=[6, 7]).contiguous()
+
+    inp = elementwise_inputs()
+    out.update({f"elementwise/in/{k}": v for k, v in inp.items()})
+    norm = r_layers.RMSNorm(256, eps=1e-5)
+    norm.weight.data = inp["w"]
+    with torch.no_grad():
+        out["elementwise/rms_norm"] = norm(inp["x"]).contiguous()
+    table = r_rope.precompute_freqs_cis(128, 1000, 1e6)
+    out["elementwise/rope_table_rows"] = torch.view_as_real(table)[ROPE_SAMPLE_ROWS].contiguous()
+    xq, xk = r_rope.apply_rotary_emb(inp["q"], inp["k"], table[inp["positions"]])
+    out["elementwise/rope_q"], out["elementwise/rope_k"] = xq.contiguous(), xk.contiguous()
+    meta = {"torch": torch.__version__, "cpu_capability": torch.backends.cpu.get_cpu_capability(),
+            "rope_table_sha256": tensor_sha256(torch.view_as_real(table)),
+            "reference": "mistralai/mistral-inference@2557e12 (v1.6.0) modules, unmodified, via oracle/ref_shims.py"}
+    return out, meta
+
+
 def main() -> None:
     GOLDEN_DIR.mkdir(parents=True, exist_ok=True)
     import safetensors.torch
@@ -155,6 +234,14 @@ def main() -> None:
         safetensors.torch.save_file(out, str(GOLDEN_DIR / "config1_7b_1layer.safetensors"), metadata=meta)
         print(f"config1_7b_1layer: seed={seed} tokens={out['tokens'].tolist()}")
         if "--config1" in sys.argv:
+            return
+
+    if "--modules" in sys.argv or "--all" in sys.argv:
+        out, meta = run_modules()
+        MODULES_FILE.parent.mkdir(parents=True, exist_ok=True)
+        safetensors.torch.save_file(out, str(MODULES_FILE), metadata=meta)
+        print(f"{MODULES_FILE.relative_to(REPO)}: {len(out)} tensors, {sum(v.numel() * v.element_size() for v in out.values())} bytes")
+        if "--modules" in sys.argv:
             return
 
     for name, case in CASES.items():

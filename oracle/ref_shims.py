@@ -7,9 +7,9 @@ cache.py:5-10, vision_encoder.py) and `simple_parsing` (args.py:4, moe.py:6, lor
 `install()` registers minimal stand-ins in `sys.modules` and puts the reference's `src/` on
 `sys.path`; after that `import mistral_inference.transformer` etc. work unmodified.
 
-Only usable where `/root/reference` exists (this container, not the GPU box): used by
-`oracle/make_golden.py` to produce tests/golden/ and by tests/test_oracle_vs_reference.py to pin
-the restatement.  Mask semantics: SURVEY.md Appendix B.
+Only usable where a checkout of the reference is installed (MISTRAL_REFERENCE_SRC): used by
+`oracle/make_golden.py` to produce tests/golden/, the fixtures that pin the restatement.  Mask
+semantics: SURVEY.md Appendix B.
 """
 import dataclasses
 import os
